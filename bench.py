@@ -6,7 +6,7 @@ Workload at every N: SlowFast-8x8-R50 eval forward, batch 8 per GPU, 3x32x224x22
 batch; weak scaling (per-GPU batch fixed), clips sharded across ranks, one NCCL all-gather of the
 [8,400] logits per step.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 Prints ONE JSON line on rank 0 (see the contract in the task statement): value = whole-job
 clips/s with inputs resident in HBM; e2e = same through the public model call with pinned HOST
@@ -155,6 +155,15 @@ def make_inputs(B, T, H, W, is_sf, seed):
     return TS.slowfast_inputs(clip) if is_sf else clip
 
 
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: write what the timed path returned in its last step as DIR/<name>.npy (float32).  Inputs and
+    weights come from fixed seeds, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def pick_cpu_threads(model, T, H, W, is_sf):
     """The reference (ATen/oneDNN conv3d) does not scale to every core of a 128-thread host at these
     sizes - pick the thread count that is actually fastest (candidates <= visible cores)."""
@@ -216,8 +225,10 @@ def run_reference(args, rank, world):
         oracle_forward(model, inp)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle_forward(model, inp)
+        out = oracle_forward(model, inp)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": out})
     v = b * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "clips/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
@@ -259,9 +270,11 @@ def run_torch_gpu(args, rank, world):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step()
+        out = step()
     e1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": out})
     ms = e0.elapsed_time(e1) / args.steps
     print(json.dumps({"impl": "torch-gpu", "metric": METRIC, "value": B / (ms / 1e3), "unit": "clips/s", "n_gpus": 1,
                       "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -292,7 +305,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--resident-only", action="store_true", help="A/B runs: time the resident step only and print a short line")
     ap.add_argument("--dump-kernels", default=None, help="write per-launch times (JSON) to this path")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the logits of the last timed step to DIR/logits.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     from pytorchvideo_b200 import parallel as PAR
@@ -364,12 +381,14 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def timed(fn, steps, drain=None):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last["out"] = fn()
         if drain is not None:
             drain()                              # every step's result is read inside the timed region
         e1.record()
@@ -390,6 +409,9 @@ def main():
     launches_before = _lib.launch_count()
     ms = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the step returns a view of the plan's static output buffer: copy it before the e2e passes below reuse the plan
+        dump_outputs(args.dump_outputs, {"logits": last["out"]})
     ms_per_step = ms / args.steps
     value = world * B * args.steps / (ms / 1e3)
 

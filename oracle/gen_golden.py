@@ -256,6 +256,26 @@ def gen_detection():
     torch.save(out, os.path.join(GOLD, "detection.pt"))
 
 
+def gen_lowering():
+    """The plans lowered from the reference's own model objects: module tree (path, class name), output shape, op
+    names and kernel-kind counts for each model, on zero inputs (the lowering reads shapes and module types only)."""
+    import pytorchvideo.models.hub as RH
+    from pytorchvideo_b200 import testing as TS
+    from pytorchvideo_b200.engine.lower import lower_only
+    out = {}
+    for name, shape in (("x3d_xs", (1, 3, 4, 160, 160)), ("slowfast_r50", (1, 3, 32, 224, 224)),
+                        ("mvit_base_16x4", (1, 3, 16, 224, 224))):
+        ref = getattr(RH, name)(pretrained=False).eval()
+        inp = TS.slowfast_inputs(torch.zeros(shape)) if name.startswith("slowfast") else torch.zeros(shape)
+        plan, out_shape = lower_only(ref, inp)
+        out[name] = {"input_shapes": [tuple(t.shape) for t in inp] if isinstance(inp, list) else [tuple(inp.shape)],
+                     "modules": [(n, type(m).__name__) for n, m in ref.named_modules()],
+                     "output_shape": tuple(out_shape), "ops": [n for n, _ in plan.ops], "stats": dict(plan.stats)}
+        print("lowering %-16s ok  %d modules, %d ops, out %s" % (name, len(out[name]["modules"]), len(plan.ops),
+                                                                  out[name]["output_shape"]), flush=True)
+    torch.save(out, os.path.join(GOLD, "lowering.pt"))
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=None)
@@ -263,6 +283,7 @@ if __name__ == "__main__":
     ap.add_argument("--skip-transforms", action="store_true")
     ap.add_argument("--skip-layers", action="store_true")
     ap.add_argument("--skip-detection", action="store_true")
+    ap.add_argument("--skip-lowering", action="store_true")
     a = ap.parse_args()
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(os.cpu_count() or 1)
@@ -272,5 +293,7 @@ if __name__ == "__main__":
         gen_layers()
     if not a.skip_detection and not a.only:
         gen_detection()
+    if not a.skip_lowering and not a.only:
+        gen_lowering()
     if not a.skip_models:
         gen_models(a.only)

@@ -210,30 +210,19 @@ def test_layer_modules_lower_on_the_host(name):
 
 def test_lowering_accepts_the_reference_modules_themselves():
     """INTEGRATION.md route 2: the lowering dispatches on the reference's class / attribute NAMES, so the reference's
-    own model objects lower to the same plan as this package's trees.  Runs where /root/reference exists (the
-    authoring container); skipped on the GPU box."""
-    import sys
-    if not os.path.isdir("/root/reference/pytorchvideo"):
-        pytest.skip("reference checkout not present")
-    shim = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "shim")
-    added = [p for p in (shim, "/root/reference") if p not in sys.path]
-    sys.path[:0] = added
-    try:
-        import pytorchvideo.models.hub as RH
-        for name, inp in (("x3d_xs", torch.zeros(1, 3, 4, 160, 160)), ("slowfast_r50", TS.slowfast_inputs(torch.zeros(1, 3, 32, 224, 224))),
-                          ("mvit_base_16x4", torch.zeros(1, 3, 16, 224, 224))):
-            ref = getattr(RH, name)(pretrained=False).eval()
-            mine = getattr(PH, name)().eval()
-            p_ref, s_ref = lower_only(ref, inp)
-            p_mine, s_mine = lower_only(mine, inp)
-            assert s_ref == s_mine
-            assert [n for n, _ in p_ref.ops] == [n for n, _ in p_mine.ops]
-            assert p_ref.stats == p_mine.stats
-    finally:
-        for p in added:
-            sys.path.remove(p)
-        for k in [k for k in sys.modules if k == "pytorchvideo" or k.startswith("pytorchvideo.") or k.startswith("fvcore")]:
-            del sys.modules[k]
+    own model objects lower to the same plan as this package's trees.  tests/golden/lowering.pt holds the reference
+    models' module trees and the plans lowered from them (oracle/gen_golden.py)."""
+    gold = torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "lowering.pt"), weights_only=False)
+    assert sorted(gold) == ["mvit_base_16x4", "slowfast_r50", "x3d_xs"]
+    for name, g in gold.items():
+        mine = getattr(PH, name)().eval()
+        assert [(n, type(m).__name__) for n, m in mine.named_modules()] == g["modules"]
+        shapes = g["input_shapes"]
+        inp = [torch.zeros(s) for s in shapes] if len(shapes) > 1 else torch.zeros(shapes[0])
+        p_mine, s_mine = lower_only(mine, inp)
+        assert tuple(s_mine) == g["output_shape"]
+        assert [n for n, _ in p_mine.ops] == g["ops"]
+        assert p_mine.stats == g["stats"]
 
 
 def test_modules_deepcopy_without_their_compiled_plans():
