@@ -84,3 +84,34 @@ def test_product_never_imports_oracle():
             if f.endswith(".py") and re.search(r"^\s*(from|import)\s+oracle\b", open(os.path.join(dp, f)).read(), re.M):
                 bad.append(f)
     assert not bad
+
+
+# Entry points that need no direct parity test of their own, with the reason.
+NO_DIRECT_GPU_TEST = {
+    "pv_abi_version": "library metadata, checked on the CPU by test_library_loads_and_exports_every_declared_symbol",
+    "pv_last_error": "error text only; every failing call in the suite reports it",
+    "pv_device_info": "device query; every GPU test calls it through _lib.require_device",
+    "pv_launch_count": "a counter; smoke() checks it grows",
+    "pv_conv3d_tcgen05_supported": "host predicate, asserted by the conv cases that pick the tensor-core route",
+    "pv_conv3d_stem_rows_supported": "host predicate, exercised by Plan.emit_conv in the stem route cases",
+    "pv_bottleneck_fused_supported": "host predicate, exercised by the lowering of the fused bottleneck block",
+    "pv_zero_f32": "a stream-ordered cudaMemsetAsync",
+    "pv_clip_transform_fwd": "single-clip transform, compared with the numpy oracle by smoke()",
+    "pv_bottleneck_fused_fwd": "covered through compile_model in test_gpu_ops.py::test_fused_bottleneck_block",
+}
+
+
+def test_every_compute_entry_point_has_a_direct_gpu_test():
+    """Every pv_* function of include/pv_b200.h is named by at least one tests/test_gpu_*.py, unless it is listed in
+    NO_DIRECT_GPU_TEST with a reason: a new entry point without a test, or a stale list entry, fails here."""
+    names = _header_functions()
+    stale = sorted(set(NO_DIRECT_GPU_TEST) - set(names))
+    assert not stale, "NO_DIRECT_GPU_TEST names functions the header no longer declares: %s" % stale
+    texts = []
+    tests_dir = os.path.join(ROOT, "tests")
+    for f in sorted(os.listdir(tests_dir)):
+        if f.startswith("test_gpu_") and f.endswith(".py"):
+            texts.append(open(os.path.join(tests_dir, f)).read())
+    untested = [n for n in names if n not in NO_DIRECT_GPU_TEST
+                and not any(re.search(r"\b%s\b" % n, t) for t in texts)]
+    assert not untested, "entry points without a direct GPU test: %s" % untested

@@ -328,3 +328,35 @@ def test_mvit_variants_lower_on_the_host(variant):
             assert sum(n.endswith(".pool_kv.dwconv") for n in names) == 4 and not any(".pool_k." in n for n in names)
         if variant == "no_kv_pool":
             assert not any(".pool_" in n and ".attn." in n for n in names)
+
+
+@pytest.mark.parametrize("stem,k,s,p,W,mutation", [
+    ("x3d_l", (1, 3, 3), (1, 2, 2), (0, 1, 1), 312, "second W tile one pixel early"),
+    ("slow", (1, 7, 7), (1, 2, 2), (0, 3, 3), 224, "corner tap zeroed"),
+    ("i3d", (5, 7, 7), (1, 2, 2), (2, 3, 3), 224, "last temporal tap zeroed"),
+])
+def test_entry_point_tolerance_detects_one_missing_tap(stem, k, s, p, W, mutation):
+    """The per-element bound of tests/test_gpu_entry_points.py accepts one f16 rounding of the float64 reference but
+    rejects the reference of a convolution with one tap missing, or with its second 128-pixel W tile shifted."""
+    from test_gpu_entry_points import conv_reference, worst_ratio
+    g = torch.Generator().manual_seed(len(stem))
+    T = 3 if k[0] > 1 else 1
+    x = TS.f16_exact(torch.randn(2, 3, T, 16, W, generator=g))
+    w = TS.f16_exact(torch.randn(24, 3, *k, generator=g) * (2.0 / (3 * k[0] * k[1] * k[2])) ** 0.5)
+    scale, bias = torch.rand(24, generator=g) + 0.5, torch.rand(24, generator=g) - 0.5
+    ref, S = conv_reference(x, w, scale, bias, s, p, act="relu")
+    assert worst_ratio(TS.f16_exact(ref.float()), ref, S, "f16") <= 1.0
+    assert worst_ratio(ref.float(), ref, S, "f32") <= 1.0
+    if mutation.startswith("second W tile"):
+        assert ref.shape[-1] == 156
+        bad = ref.clone()
+        bad[..., 128:] = ref[..., 127:-1]
+    else:
+        w2 = w.clone()
+        if mutation == "corner tap zeroed":
+            w2[:, :, 0, -1, -1] = 0
+        else:
+            w2[:, :, -1] = 0
+        bad, _ = conv_reference(x, w2, scale, bias, s, p, act="relu")
+    for dt in ("f16", "f32"):
+        assert worst_ratio(bad, ref, S, dt) > 4.0, (mutation, dt)
